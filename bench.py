@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the batched physics step on humanoid.xml (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--nworld 8192]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--nworld 8192] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], reference benchmarks/humanoid/__init__.py): humanoid, nworld=8192 per GPU, nconmax=24,
@@ -44,7 +44,12 @@ def parse():
   p.add_argument("--no-graph", action="store_true", help="launch kernels directly instead of replaying a CUDA graph")
   p.add_argument("--cpu-sample-worlds", type=int, default=None)
   p.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (kernel A/B sweeps)")
-  return p.parse_args()
+  p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                 help="after the timed steps, write the Data arrays of the last one as DIR/<name>.npy (a fixed world sample, at most 64 MB)")
+  a = p.parse_args()
+  if a.steps < 1 or a.warmup < 0:
+    p.error("--steps must be >= 1 and --warmup >= 0")
+  return a
 
 
 def usable_cores() -> int:
@@ -211,6 +216,47 @@ def run_reference(args):
 
 # --------------------------------------------------------------------------------------------- GPU arm
 
+DUMP_BYTES = 60 * 2**20  # array payload; with the .npy headers the dump stays below 64 MB however a megabyte is counted
+
+
+def dump_outputs(d, out_dir, seed=0):
+  """Writes the Data arrays a caller of the step receives as out_dir/<name>.npy: the top-level and efc_* fields of a fixed, seeded
+  sample of worlds (all of them when they fit DUMP_BYTES), and the contact_* fields of those worlds' contacts, grouped by world in
+  pool order (at most nconmax per sampled world on average).  Float fields stay float32; integer fields are written as float64
+  (exact).  worlds.npy lists the sampled world ids.  The sample depends on the sizes only, so two builds dump the same worlds."""
+  import torch
+
+  nworld = d.nworld
+  per_world = {("efc_" if s is d.efc else "") + k: v for s in (d, d.efc) for k, v in vars(s).items()
+               if isinstance(v, torch.Tensor) and v.dim() and v.shape[0] == nworld and v.numel() and not k.startswith("_")}
+  nacon = min(int(d.nacon[0]), d.naconmax)
+  contact = {"contact_" + k: v[:nacon] for k, v in vars(d.contact).items() if isinstance(v, torch.Tensor) and v.dim() and v.shape[0] == d.naconmax}
+  row = lambda v: (4 if v.dtype == torch.float32 else 8) * v[0].numel()  # bytes of one world's / contact's entry as written
+  world_bytes = 8 + sum(row(v) for v in per_world.values()) + d.nconmax * sum(row(v) for v in contact.values())
+  k = max(1, min(nworld, DUMP_BYTES // world_bytes))
+  worlds = np.sort(np.random.default_rng(seed).choice(nworld, k, replace=False)) if k < nworld else np.arange(nworld)
+  idx = torch.from_numpy(worlds).to(d.qpos.device)
+  out = {"worlds": worlds.astype(np.float64)}
+  out.update({n: v.index_select(0, idx) for n, v in per_world.items()})
+  wid = d.contact.worldid[:nacon].long()
+  keep = torch.nonzero(torch.isin(wid, idx)).squeeze(1)
+  keep = keep[torch.argsort(wid[keep], stable=True)][: k * d.nconmax]  # grouped by world, pool order inside a world
+  out.update({n: v[keep] for n, v in contact.items()})
+  # the efc_id of a contact row is a contact-pool slot, and worlds claim slots in no fixed order: it is written as the contact's
+  # index within its world (as listed in contact_*), -1 on rows past nefc
+  from mujoco_warp_b200._src import constants as C
+
+  local = torch.full((max(nacon, 1),), -1, dtype=torch.long, device=wid.device)
+  local[keep] = torch.arange(len(keep), device=wid.device) - torch.searchsorted(wid[keep], wid[keep])
+  efc_id, efc_type = out["efc_id"].long(), out["efc_type"]
+  live = torch.arange(efc_id.shape[1], device=efc_id.device)[None, :] < out["nefc"][:, None]
+  is_contact = (efc_type >= C.CNSTR_CONTACT_FRICTIONLESS) & (efc_type <= C.CNSTR_CONTACT_ELLIPTIC)
+  out["efc_id"] = torch.where(is_contact, torch.where(live, local[efc_id.clamp(0, max(nacon - 1, 0))], -1), efc_id)
+  os.makedirs(out_dir, exist_ok=True)
+  for n, v in out.items():
+    a = v.cpu().numpy() if isinstance(v, torch.Tensor) else v
+    np.save(os.path.join(out_dir, n + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
 
 def run_ours(args):
   import torch
@@ -251,7 +297,18 @@ def run_ours(args):
   stream = torch.cuda.Stream()
   graph = None
   step_idx = [0]
-  initial = {n: getattr(d, n).clone() for n in ("qpos", "qvel", "ctrl", "qacc_warmstart", "time", "qacc")}
+  # every Data array, efc_* rows past nefc and accumulated overflow bits included: restoring all of them makes the Data the timed
+  # window starts from (and so every array it leaves) independent of how many untimed steps ran before
+  arrays = list({id(t): t for o in (d, d.efc, d.contact) for t in vars(o).values() if isinstance(t, torch.Tensor)}.values())
+
+  def snapshot():
+    return [t.clone() for t in arrays]
+
+  def restore(snap):
+    for t, v in zip(arrays, snap):
+      t.copy_(v)
+
+  initial = snapshot()
 
   def set_ctrl():
     if traj is not None:  # trajectory replay, zero-order hold (cli.py:154-158): every world gets the step's control row
@@ -277,17 +334,10 @@ def run_ours(args):
       with torch.cuda.graph(g, stream=stream):
         mjw.step(m, d)
       graph = g
-    # The simulated state inside the timed window is deterministic: the state is put back to the keyframe after graph capture,
+    # The simulated state inside the timed window is deterministic: the Data is put back to its put_data state after graph capture,
     # advanced by exactly `warmup` steps, snapshotted, and restored right before the timed region.  nvidia-smi needs a few hundred
     # ms before its first row, so the same load keeps running (on the live state) until it reports; those extra steps are undone
     # by the restore.
-    def snapshot():
-      return {n: getattr(d, n).clone() for n in ("qpos", "qvel", "ctrl", "qacc_warmstart", "time", "qacc")}
-
-    def restore(snap):
-      for n, v in snap.items():
-        getattr(d, n).copy_(v)
-
     restore(initial)
     step_idx[0] = 0
     sampler = ClockSampler(local)
@@ -325,6 +375,8 @@ def run_ours(args):
       stream.synchronize()
       ms = sum(a.elapsed_time(b) for a, b in evs)
     barrier()
+    if args.dump_outputs and rank == 0:
+      dump_outputs(d, args.dump_outputs)
     # ---- statistics of the run (untimed), taken from the last timed step
     ncon_mean = float(d.nacon.cpu()[0]) / nworld
     nefc_mean = float(d.nefc.float().mean().cpu())

@@ -293,7 +293,6 @@ def test_mixed_scene_forward_and_rollout(mixed):
   assert mismatched <= 10, mismatched
 
 
-@pytest.mark.xfail(strict=False, reason="added after the round's GPU minutes were spent: it has not run on a B200 yet, so it may not turn the suite red; expected to pass")
 def test_more_than_32_contacts_in_one_world(built):
   """The contact-row builder of k_constraint works in batches of 32 contacts (phase A: lane = contact, phase C: lane = row of the batch):
   a rigid rake of 40 spheres on a plane gives 40 contacts per world with 1, 4 and 6 rows per contact (contact dimensions 1, 3, 4), i.e. a

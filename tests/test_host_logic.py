@@ -84,14 +84,11 @@ def test_product_package_never_imports_oracle():
         assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, re.M), f
 
 
-def test_mjcf_compiler_matches_fixture(mjm):
-  """When the reference tree is mounted, compiling its XML reproduces the committed .npz fixture exactly."""
+def test_mjcf_compiler_matches_fixture(mjm, tmp_path):
+  """Compiling the reference's humanoid.xml reproduces the committed .npz fixture exactly."""
   from mujoco_warp_b200._src import mjcf
 
-  xml = "/root/reference/benchmarks/humanoid/humanoid.xml"
-  if not os.path.exists(xml):
-    pytest.skip("reference tree not mounted (GPU box)")
-  a = mjcf.load(xml)
+  a = mjcf.load(os.path.join(util.reference_models(tmp_path), "benchmarks", "humanoid", "humanoid.xml"))
   for k in ("body_mass", "body_inertia", "body_ipos", "body_iquat", "geom_size", "geom_pos", "geom_quat", "jnt_range", "dof_invweight0", "body_invweight0", "key_qpos", "M_colind"):
     np.testing.assert_array_equal(np.asarray(getattr(a, k)), np.asarray(getattr(mjm, k)), err_msg=k)
 

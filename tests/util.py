@@ -7,6 +7,18 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 from mujoco_warp_b200.scenes import DATA as SCENES, G1, G1_TRAJ, HUMANOID, THREE_HUMANOIDS  # noqa: E402,F401
 
+REFERENCE_MODELS = os.path.join(ROOT, "tests", "golden", "reference_models.tar.xz")
+
+
+def reference_models(dest):
+  """Unpacks the reference's MJCF model files (tools/make_reference_models.py) under `dest`, keeping their relative layout so that
+  <include> and mesh paths resolve; returns `dest`."""
+  import tarfile
+
+  with tarfile.open(REFERENCE_MODELS) as tar:
+    tar.extractall(dest, filter="data")
+  return str(dest)
+
 
 def seeded_state(mjm, nworld, key=0, seed=42, qpos_noise=0.05, qvel_noise=0.5, ctrl_noise=0.5, exact_world0=True):
   """Per-world states around a keyframe, like the reference fixture's seeded uniform noise (test_data/__init__.py:82-98)."""
